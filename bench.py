@@ -2,6 +2,7 @@
 """bench.py -- Wilson-Dslash GFLOPS / HBM GB/s on a 32^4 local volume (BASELINE.json metric).
 
   python bench.py --gpus N --steps K --warmup W            our arm (libquda_b200.so on B200)
+  python bench.py ... --dump-outputs DIR                   also save what the last of the K timed steps computed (DIR/out.npy)
   python bench.py --impl reference ...                     the reference's CPU dslash (oracle/_ref) on host cores
   python bench.py --sweep                                  (dev) launch-geometry sweep, writes gpurun_out/sweep.json
 
@@ -64,7 +65,14 @@ def parse():
                     help="(N>1) process grid (x y z t), product = N; default splits t, then z, then y.  BASELINE config 4's "
                          "2x1x1x1 is --grid 2 1 1 1 (the strided x face)")
     ap.add_argument("--no-halo-check", action="store_true", help="(N>1) skip the partitioned-vs-global-oracle parity check")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the output spinor(s) of the last one to DIR/<name>.npy (see dump_outputs)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.op == "cg" or a.sweep):
+        ap.error("--dump-outputs applies to the timed Dslash of --impl b200 (--op wilson or clover_pc)")
+    return a
 
 
 def measured_peaks():
@@ -392,6 +400,9 @@ def run_b200(a):
         ev1.record()
         barrier()
         launches = lib.b200_launch_count()
+        if a.dump_outputs:
+            # copied now: the loops below write to the same buffers (the multi-RHS line with another kernel)
+            last = [d.buf.clone() for d in (dsts if nsrc > 1 else [pairs[(rot[0] - 1) % NROT][1]])]
         # the timed region above lasts only K x ~55 us, far below nvidia-smi's sampling period: keep the identical
         # kernel running for ~1.5 s more so that the clock / throttle record covers this very workload, and report
         # its (power-capped) steady-state step time next to the K-step figure
@@ -512,6 +523,8 @@ def run_b200(a):
             out["cpu_baseline"] = info
         except Exception as e:  # the checker is optional for the measurement itself
             out["cpu_baseline"] = {"value": None, "error": str(e)}
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, "out" if world == 1 else f"out_rank{rank}", last, prec, Vh, DUMP_BYTES // world)
     if rank == 0:
         print(json.dumps(out))
     if world > 1:
@@ -585,6 +598,26 @@ def new_spinor(P, seed=None):
             dt = torch.float64 if ref.prec == 8 else torch.float32
             buf = torch.rand(ref.buf.numel() * ref.buf.element_size() // ref.prec, dtype=dt, device="cuda", generator=g).view(torch.uint8)
     return D.ColorSpinorField(buf, ref.X, ref.prec, ref.n_parity)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, name, bufs, prec, Vh, budget):
+    """--dump-outputs: native single-parity spinor buffers -> path/<name>.npy, shape [len(bufs),] Vh x 4 x 3 x 2 in the
+    precision's real type (float64 for double, float32 otherwise), spin and colour as stored (no basis rotation).  Above
+    `budget` bytes: a fixed sample of sites (seed 0) from all buffers together, shape n x 4 x 3 x 2, the same at every run."""
+    import numpy as np
+    from quda_b200 import fields as F
+    arr = np.stack([F.spinor_from_native(b.cpu().numpy(), Vh, prec, rotate=False).astype(F.real_dtype(prec)) for b in bufs])
+    sites = arr.reshape(-1, 4, 3, 2)
+    keep = budget // sites[0].nbytes
+    if len(sites) > keep:
+        arr = sites[np.sort(np.random.default_rng(0).choice(len(sites), keep, replace=False))]
+    elif len(bufs) == 1:
+        arr = arr[0]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, name + ".npy"), arr)
 
 
 def multi_rhs_line(a, P, D, L, stream, prec, Vh, peak, nsrc=8, steps=50):

@@ -6,8 +6,9 @@ Two shared objects live here (both built by ``oracle/Makefile``; ``__graft_entry
   (``tests/host_reference/wilson_dslash_reference.cpp``, ``clover_reference.cpp``, field generators of
   ``tests/utils/host_utils.cpp``), used as the checker in ``tests/`` and as the CPU baseline.
 * ``_ref/libquda_hostref.so``  -- the reference's *own* host sources compiled in place
-  (``ref_glue.cpp`` only supplies link-time stand-ins); used to pin the restatement
-  (``tests/test_oracle_pin.py``) and as ``cpu_baseline.kind == "reference"`` in ``bench.py``.
+  (``ref_glue.cpp`` only supplies link-time stand-ins); records the outputs that pin the restatement
+  (``tests/golden/oracle_pin.json``, see ``tests/test_oracle_pin.py``) and is ``cpu_baseline.kind == "reference"`` in
+  ``bench.py``.
 
 Only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py`` (cpu_baseline / ``--impl reference``) may
 import this package.  ``quda_b200`` never does; it fails loudly without its CUDA library instead.

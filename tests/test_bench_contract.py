@@ -49,6 +49,39 @@ def test_torchrun_ranks_are_never_pinned():
         assert out.stdout.split() == ["None", "None"], out.stdout
 
 
+def test_dump_outputs(tmp_path):
+    """--dump-outputs: native buffers back in [site][spin][colour][re,im] order in the precision's real type, and above the
+    byte budget the same seeded sample of sites at every call"""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    from quda_b200 import fields as F
+    Vh = 64
+    host = [np.random.default_rng(i).random((Vh, 4, 3, 2)) for i in range(3)]
+    for prec, dt in ((8, np.float64), (4, np.float32), (2, np.float32)):
+        bufs = [torch.from_numpy(F.spinor_to_native(h, prec, rotate=False)) for h in host]
+        bench.dump_outputs(str(tmp_path), "one", bufs[:1], prec, Vh, bench.DUMP_BYTES)
+        one = np.load(tmp_path / "one.npy")
+        assert one.dtype == dt and one.shape == (Vh, 4, 3, 2)
+        assert np.array_equal(one, F.spinor_from_native(bufs[0].numpy(), Vh, prec, rotate=False))
+        bench.dump_outputs(str(tmp_path), "all", bufs, prec, Vh, bench.DUMP_BYTES)
+        assert np.load(tmp_path / "all.npy").shape == (3, Vh, 4, 3, 2)
+        budget = 50 * 24 * np.dtype(dt).itemsize
+        samples = []
+        for _ in range(2):
+            bench.dump_outputs(str(tmp_path), "sample", bufs, prec, Vh, budget)
+            samples.append(np.load(tmp_path / "sample.npy"))
+        assert samples[0].shape == (50, 4, 3, 2) and samples[0].nbytes <= budget
+        assert np.array_equal(samples[0], samples[1])
+
+
+def test_dump_outputs_and_steps_are_checked():
+    for args in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "d"], ["--op", "cg", "--dump-outputs", "d"]):
+        r = _run(args)
+        assert r.returncode == 2 and "error" in r.stderr, (args, r.stderr[-1000:])
+
+
 def test_process_grid_defaults():
     sys.path.insert(0, ROOT)
     import bench
