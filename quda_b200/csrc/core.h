@@ -297,6 +297,66 @@ namespace b200
   }
   template <typename T> B2_HD cplx<T> conj(const cplx<T> &a) { return {a.re, -a.im}; }
 
+  // ------------------------------------------------------------------ paired FP32 (sm_100: FFMA2 / FADD2 / FMUL2)
+  // One instruction does the same fp32 operation on both halves of a 64-bit register pair, each lane rounded exactly as the
+  // scalar instruction.  The fp32 site code (fp32 storage, and half, which computes in fp32) runs its complex arithmetic on
+  // (re, im) pairs through these helpers, keeping every lane's operation sequence and FMA contraction of the scalar code,
+  // so the output is bit-identical to the scalar path (B2_PACKED_F32=0, also what the host twin and fp64 compile).
+  //
+  // What ptxas folds into operand modifiers at no cost: swapping the halves (`.LO_HI`), negating one half (`.NP`) or
+  // both, and a scalar broadcast (`R.F32`) for the second factor when it is written as pack2(x, x) or pack2(-x, x).  So
+  // multiplying by +-i is fma2(swap2(h), pack2(-x, x), acc): the sign pattern goes on the pair, the scalar is broadcast.
+  // ptxas contracts a mul2 feeding an add2 into one FFMA2 despite the .rn, so a product that the scalar code rounds
+  // before adding is only ever used as a multiplicand or as the addend of an fma2.
+#ifndef B2_PACKED_F32
+#define B2_PACKED_F32 1
+#endif
+#if defined(__CUDA_ARCH__) && B2_PACKED_F32
+#define B2_F32X2 1
+  using f32x2 = unsigned long long;
+  B2_D f32x2 pack2(float lo, float hi)
+  {
+    f32x2 r;
+    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
+    return r;
+  }
+  B2_D void unpack2(f32x2 p, float &lo, float &hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(p)); }
+  B2_D f32x2 fma2(f32x2 a, f32x2 b, f32x2 c)
+  {
+    f32x2 d;
+    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
+    return d;
+  }
+  B2_D f32x2 add2(f32x2 a, f32x2 b)
+  {
+    f32x2 d;
+    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
+    return d;
+  }
+  B2_D f32x2 sub2(f32x2 a, f32x2 b)
+  {
+    f32x2 d;
+    asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
+    return d;
+  }
+  B2_D f32x2 mul2(f32x2 a, f32x2 b)
+  {
+    f32x2 d;
+    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
+    return d;
+  }
+  B2_D f32x2 swap2(f32x2 a)
+  {
+    float lo, hi;
+    unpack2(a, lo, hi);
+    return pack2(hi, lo);
+  }
+  B2_D f32x2 ld2(const float *p) { return pack2(p[0], p[1]); }
+  B2_D void st2(float *p, f32x2 v) { unpack2(v, p[0], p[1]); }
+#else
+#define B2_F32X2 0
+#endif
+
   // ------------------------------------------------------------------ lattice geometry + index math
   struct Geom {
     int X[4];    // local lattice extents (full sites), X[0] even
@@ -570,18 +630,7 @@ namespace b200
       } else if constexpr (recon == 12) {
 #pragma unroll
         for (int i = 0; i < 12; i++) u[i] = t[i];
-        const real s = u0(dir, x_cb);
-        // row2 = u0 * conj(row0 x row1)
-        const cplx<real> a0 {u[0], u[1]}, a1 {u[2], u[3]}, a2 {u[4], u[5]};
-        const cplx<real> b0 {u[6], u[7]}, b1 {u[8], u[9]}, b2 {u[10], u[11]};
-        cplx<real> c0 = cmul(a1, b2), c1 = cmul(a2, b0), c2 = cmul(a0, b1);
-        const cplx<real> d0 = cmul(a2, b1), d1 = cmul(a0, b2), d2_ = cmul(a1, b0);
-        u[12] = s * (c0.re - d0.re);
-        u[13] = -s * (c0.im - d0.im);
-        u[14] = s * (c1.re - d1.re);
-        u[15] = -s * (c1.im - d1.im);
-        u[16] = s * (c2.re - d2_.re);
-        u[17] = -s * (c2.im - d2_.im);
+        row2(u, u0(dir, x_cb));
       } else {
         unpack8(u, t, u0(dir, x_cb));
       }
@@ -608,20 +657,40 @@ namespace b200
         } else {
 #pragma unroll
           for (int i = 0; i < 12; i++) u[i] = t[i];
-          const real s = u0(dir, x_cb) * kFixedInvMax;
-          const cplx<real> a0 {u[0], u[1]}, a1 {u[2], u[3]}, a2 {u[4], u[5]};
-          const cplx<real> b0 {u[6], u[7]}, b1 {u[8], u[9]}, b2 {u[10], u[11]};
-          cplx<real> c0 = cmul(a1, b2), c1 = cmul(a2, b0), c2 = cmul(a0, b1);
-          const cplx<real> d0 = cmul(a2, b1), d1 = cmul(a0, b2), d2_ = cmul(a1, b0);
-          u[12] = s * (c0.re - d0.re);
-          u[13] = -s * (c0.im - d0.im);
-          u[14] = s * (c1.re - d1.re);
-          u[15] = -s * (c1.im - d1.im);
-          u[16] = s * (c2.re - d2_.re);
-          u[17] = -s * (c2.im - d2_.im);
+          row2(u, u0(dir, x_cb) * kFixedInvMax);
           scale = kFixedInvMax;
         }
       }
+    }
+
+    // recon-12: row 2 = s * conj(row0 x row1), rows 0 and 1 already in u[0..11]
+    B2_HD static void row2(real *u, real s)
+    {
+#if B2_F32X2
+      if constexpr (std::is_same<real, float>::value) {
+        // cmul(a, b) as nvcc contracts it: re = fma(a.re, b.re, -(a.im*b.im)), im = fma(a.im, b.re, a.re*b.im)
+        auto cmul2 = [](f32x2 a, const float *b) {
+          return fma2(a, pack2(b[0], b[0]), mul2(swap2(a), pack2(-b[1], b[1])));
+        };
+        const f32x2 a0 = ld2(u), a1 = ld2(u + 2), a2 = ld2(u + 4);
+        const float *b0 = u + 6, *b1 = u + 8, *b2 = u + 10;
+        const f32x2 ss = pack2(s, -s);
+        st2(u + 12, mul2(sub2(cmul2(a1, b2), cmul2(a2, b1)), ss));
+        st2(u + 14, mul2(sub2(cmul2(a2, b0), cmul2(a0, b2)), ss));
+        st2(u + 16, mul2(sub2(cmul2(a0, b1), cmul2(a1, b0)), ss));
+        return;
+      }
+#endif
+      const cplx<real> a0 {u[0], u[1]}, a1 {u[2], u[3]}, a2 {u[4], u[5]};
+      const cplx<real> b0 {u[6], u[7]}, b1 {u[8], u[9]}, b2 {u[10], u[11]};
+      cplx<real> c0 = cmul(a1, b2), c1 = cmul(a2, b0), c2 = cmul(a0, b1);
+      const cplx<real> d0 = cmul(a2, b1), d1 = cmul(a0, b2), d2_ = cmul(a1, b0);
+      u[12] = s * (c0.re - d0.re);
+      u[13] = -s * (c0.im - d0.im);
+      u[14] = s * (c1.re - d1.re);
+      u[15] = -s * (c1.im - d1.im);
+      u[16] = s * (c2.re - d2_.re);
+      u[17] = -s * (c2.im - d2_.im);
     }
 
     // load link (dir, x_cb, parity) into row-major u[18] = U[row][col] (re, im)
@@ -748,6 +817,27 @@ namespace b200
   // h: 2 spins x 3 colours (12 reals, (s*3+c)*2+reim); u row-major.  r = U h  or  r = U^dagger h.
   template <bool adjoint, typename real> B2_HD void su3_mul(real *r, const real *u, const real *h)
   {
+#if B2_F32X2
+    if constexpr (std::is_same<real, float>::value) { // per lane the chain below: (re, im) += ur (hr, hi) + ui (-hi, hr)
+#pragma unroll
+      for (int s = 0; s < 2; s++) {
+#pragma unroll
+        for (int i = 0; i < 3; i++) {
+          f32x2 acc = pack2(0.0f, 0.0f);
+#pragma unroll
+          for (int j = 0; j < 3; j++) {
+            const float ur = adjoint ? u[(j * 3 + i) * 2] : u[(i * 3 + j) * 2];
+            const float ui = adjoint ? -u[(j * 3 + i) * 2 + 1] : u[(i * 3 + j) * 2 + 1];
+            const f32x2 hv = ld2(h + (s * 3 + j) * 2);
+            acc = fma2(hv, pack2(ur, ur), acc);
+            acc = fma2(swap2(hv), pack2(-ui, ui), acc);
+          }
+          st2(r + (s * 3 + i) * 2, acc);
+        }
+      }
+      return;
+    }
+#endif
 #pragma unroll
     for (int s = 0; s < 2; s++) {
 #pragma unroll
@@ -775,6 +865,34 @@ namespace b200
   template <typename real> B2_HD void project(real *h, const real *v, int mu, int sign)
   {
     const real sg = (real)sign;
+#if B2_F32X2
+    if constexpr (std::is_same<real, float>::value) { // the +-1 factors are exact: fma2 by them is the scalar FADD
+      const f32x2 pi = pack2(-sg, sg), mi = pack2(sg, -sg), p1 = pack2(sg, sg), m1 = pack2(-sg, -sg); // +-s*i, +-s
+#pragma unroll
+      for (int c = 0; c < 3; c++) {
+        const f32x2 v0 = ld2(v + (0 * 3 + c) * 2), v1 = ld2(v + (1 * 3 + c) * 2);
+        const f32x2 v2 = ld2(v + (2 * 3 + c) * 2), v3 = ld2(v + (3 * 3 + c) * 2);
+        f32x2 h0, h1;
+        if (mu == 0) {
+          h0 = fma2(swap2(v3), pi, v0);
+          h1 = fma2(swap2(v2), pi, v1);
+        } else if (mu == 1) {
+          h0 = fma2(v3, p1, v0);
+          h1 = fma2(v2, m1, v1);
+        } else if (mu == 2) {
+          h0 = fma2(swap2(v2), pi, v0);
+          h1 = fma2(swap2(v3), mi, v1);
+        } else {
+          const f32x2 two = pack2(2.0f, 2.0f);
+          h0 = mul2(sign > 0 ? v0 : v2, two);
+          h1 = mul2(sign > 0 ? v1 : v3, two);
+        }
+        st2(h + (0 * 3 + c) * 2, h0);
+        st2(h + (1 * 3 + c) * 2, h1);
+      }
+      return;
+    }
+#endif
 #pragma unroll
     for (int c = 0; c < 3; c++) {
       const real v0r = v[(0 * 3 + c) * 2], v0i = v[(0 * 3 + c) * 2 + 1];
@@ -817,10 +935,61 @@ namespace b200
     }
   }
 
+#if B2_F32X2
+  // acc += s * reconstruct(h) on (re, im) pairs: one FFMA2 per colour and spin, as the scalar forms below
+  B2_D void reconstruct_add_x2(float *acc, const float *h, int mu, int sign, float s)
+  {
+    const float sg = (float)sign * s;
+    const f32x2 p = pack2(s, s), ps = pack2(sg, sg), ms = pack2(-sg, -sg), pi = pack2(sg, -sg), mi = pack2(-sg, sg);
+#pragma unroll
+    for (int c = 0; c < 3; c++) {
+      const f32x2 h0 = ld2(h + (0 * 3 + c) * 2), h1 = ld2(h + (1 * 3 + c) * 2);
+      float *a0 = acc + (0 * 3 + c) * 2, *a1 = acc + (1 * 3 + c) * 2, *a2 = acc + (2 * 3 + c) * 2, *a3 = acc + (3 * 3 + c) * 2;
+      if (mu == 3 && sign < 0) {
+        st2(a2, fma2(h0, p, ld2(a2)));
+        st2(a3, fma2(h1, p, ld2(a3)));
+        continue;
+      }
+      st2(a0, fma2(h0, p, ld2(a0)));
+      st2(a1, fma2(h1, p, ld2(a1)));
+      if (mu == 0) { // rows 2,3: -s*i*h1, -s*i*h0
+        st2(a2, fma2(swap2(h1), pi, ld2(a2)));
+        st2(a3, fma2(swap2(h0), pi, ld2(a3)));
+      } else if (mu == 1) { // rows 2,3: -s*h1, +s*h0
+        st2(a2, fma2(h1, ms, ld2(a2)));
+        st2(a3, fma2(h0, ps, ld2(a3)));
+      } else if (mu == 2) { // rows 2,3: -s*i*h0, +s*i*h1
+        st2(a2, fma2(swap2(h0), pi, ld2(a2)));
+        st2(a3, fma2(swap2(h1), mi, ld2(a3)));
+      }
+    }
+  }
+#endif
+
+  // h = 2 t (12 reals): the t-direction projection of a spin pair that is already loaded
+  template <typename real> B2_HD void twice12(real *h, const real *t)
+  {
+#if B2_F32X2
+    if constexpr (std::is_same<real, float>::value) {
+#pragma unroll
+      for (int i = 0; i < 12; i += 2) st2(h + i, mul2(ld2(t + i), pack2(2.0f, 2.0f)));
+      return;
+    }
+#endif
+#pragma unroll
+    for (int i = 0; i < 12; i++) h[i] = 2 * t[i];
+  }
+
   // acc += reconstruct(h) for P(mu, sign)
   template <typename real> B2_HD void reconstruct_add(real *acc, const real *h, int mu, int sign)
   {
     const real sg = (real)sign;
+#if B2_F32X2
+    if constexpr (std::is_same<real, float>::value) {
+      reconstruct_add_x2(acc, h, mu, sign, 1.0f); // a += 1 * h is the scalar FADD
+      return;
+    }
+#endif
 #pragma unroll
     for (int c = 0; c < 3; c++) {
       const real h0r = h[(0 * 3 + c) * 2], h0i = h[(0 * 3 + c) * 2 + 1];
@@ -851,6 +1020,12 @@ namespace b200
   // acc += s * reconstruct(h): the deferred-scaling form (one FFMA per component instead of FADD + earlier FMULs)
   template <typename real> B2_HD void reconstruct_add_scaled(real *acc, const real *h, int mu, int sign, real s)
   {
+#if B2_F32X2
+    if constexpr (std::is_same<real, float>::value) {
+      reconstruct_add_x2(acc, h, mu, sign, s);
+      return;
+    }
+#endif
     const real sg = (real)sign * s;
 #pragma unroll
     for (int c = 0; c < 3; c++) {

@@ -209,8 +209,7 @@ namespace b200
     } else if (d == 3) {
       real t[12];
       load_spin_pair<P, (sign > 0)>(t, in, n_cb);
-#pragma unroll
-      for (int i = 0; i < 12; i++) h[i] = 2 * t[i];
+      twice12(h, t);
     } else {
       real v[24];
       in.load(v, n_cb);
@@ -533,8 +532,7 @@ namespace b200
         if (d == 3) {
           real t[12];
           load_spin_pair<P, (sign > 0)>(t, in, n_cb);
-#pragma unroll
-          for (int i = 0; i < 12; i++) h[i] = 2 * t[i];
+          twice12(h, t);
         } else {
           real v[24];
           in.load(v, n_cb);

@@ -535,8 +535,7 @@ namespace b200
       constexpr int np = 12 / P::Ns;
       real t[12];
       lds_planes<P, (sign > 0) ? 0 : np, np>(t, spinor_rec, srow_bytes);
-#pragma unroll
-      for (int i = 0; i < 12; i++) h[i] = 2 * t[i];
+      twice12(h, t);
     } else {
       real v[24];
       lds_planes<P, 0, 24 / P::Ns>(v, spinor_rec, srow_bytes);
